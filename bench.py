@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- candidate-train examples/sec per AdaNet iteration (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one training step of EVERY candidate of the iteration on one
 minibatch (subnetwork fwd+bwd+update, candidate-ensemble head, EMA).  Workload
@@ -22,6 +22,10 @@ batch and a D2H read of every step's losses (an `after_run` hook) inside the tim
 clock samples; `roofline` carries the measured cuBLAS peak of the MMA kind the kernel issues
 beside the bf16 peak of MEASURED_PEAKS.json; `cpu_baseline` = the faster of two CPU restatements
 (NumPy/OpenBLAS oracle, torch-CPU oneDNN port) on the full B=32768 minibatch.
+
+`--dump-outputs DIR` writes, after the K timed steps, what the last of them computed (see dump_outputs) as .npy
+files, so that two builds can be compared output for output: data and initial weights are seeded, so the same
+arguments give the same inputs.  The benchmark writes nothing into the source tree; it runs the library build() made.
 """
 
 import argparse
@@ -36,6 +40,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ in the (possibly read-only) source tree
 
 WIDTHS = (64, 128, 192, 256, 384, 512, 768, 1024)
 IN_DIM, CLASSES, BATCH = 100, 10, 32768
@@ -338,6 +343,28 @@ def measure_dominant_kernel(lib, torch, reps=20):
   return float(np.mean(times)), 2.0 * B * I * O, "tcgen05_3x%s_planes" % fmt
 
 
+def dump_outputs(plan, out_dir):
+  """What the plan's most recent train_step computed, per candidate this rank reports, as `<name>.<array>.npy`:
+  the subnetwork weights and biases (w<i>, b<i>), mixture weights (mix<i>), ensemble bias and EMA state after the step
+  (CandidatePlan.state_dict, which also holds any optimizer slots), the step's subnetwork logits [B, C] and its loss
+  row [sub, ensemble, adanet, EMA].  Float32 (integer step counters as float64); about 21 MB for the 8-candidate
+  workload.  A row-sharded candidate
+  (N > 1) has no logits file: each of its ranks holds only its rows."""
+  os.makedirs(out_dir, exist_ok=True)
+  row = (plan.steps_done - 1) % plan.trace_capacity
+  for c in plan.candidates:
+    if not plan._reports(c.ehead):
+      continue
+    arrays = c.state_dict()
+    arrays["losses"] = arrays.pop("trace")[row]
+    if c.comm is None:
+      arrays["logits"] = c.net.logits.cpu().numpy()
+    for key, a in arrays.items():
+      a = np.asarray(a)
+      np.save(os.path.join(out_dir, "%s.%s.npy" % (c.spec.name, key)),
+              a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
+
 def _finish(world):
   """Leaves a multi-rank job without tearing the NCCL communicators down one rank at a time: ranks other than 0 finish
   long before rank 0 (which still measures the roofline kernel and cuBLAS peaks), and destroying a sub-communicator
@@ -365,8 +392,6 @@ def run_ours(args):
   torch.cuda.set_device(local)
   if world > 1:
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-  import __graft_entry__ as g
-  g.build()
   from adanet_b200 import _lib
   from adanet_b200.core import engine as eng
   from adanet_b200.core import search as srch
@@ -422,6 +447,8 @@ def run_ours(args):
   value = BATCH * args.steps / secs
   local_losses = plan.last_losses()
   assert np.isfinite(local_losses).all(), "non-finite loss in the timed region"
+  if args.dump_outputs:
+    dump_outputs(plan, args.dump_outputs)
   # ---------------- steady state: the same loop for >= 2.5 s (the chip reaches its power cap) ----------------
   sustained = None
   if not args.profile and args.sustain_seconds > 0:
@@ -616,7 +643,13 @@ def main():
   ap.add_argument("--profile", action="store_true", help="step loop only (for ncu captures)")
   ap.add_argument("--sustain-seconds", type=float, default=2.5,
                   help="length of the additional steady-state measurement (0 = skip)")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="write what the last timed step computed to DIR/<name>.npy")
   args = ap.parse_args()
+  if args.steps < 1 or args.warmup < 0:
+    ap.error("--steps must be at least 1 and --warmup at least 0")
+  if args.dump_outputs and args.impl != "ours":
+    ap.error("--dump-outputs writes the outputs of --impl ours")
   if args.impl == "reference":
     run_reference(args)
   else:

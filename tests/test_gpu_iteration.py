@@ -224,6 +224,40 @@ def test_bench_workload_parity_full_batch(built_lib):
 
 
 @pytest.mark.gpu
+def test_bench_dump_outputs_hold_the_last_step(built_lib, tmp_path):
+  """bench.py --dump-outputs writes the plan's state after its last step, that step's loss row and the logits of
+  its forward pass: the subnetwork loss recomputed from the dumped logits and labels is the dumped one."""
+  import bench
+  from adanet_b200.core import engine as eng
+  from adanet_b200.core import search as srch
+  B, D, C, steps = 256, 100, 10, 3
+  x, y = orc.make_tabular(B * 4, D, C, seed=5)
+  s = srch.AdaNetSearch(lambda t, frozen: pu.make_specs([(1, 64), (2, 128)], D, C, t, ("sgd", 0.05))[1],
+                        eng.EnsemblerPlanSpec(**ENS), D, C, B, keep_traces=False)
+  plan = s.build_iteration()
+  batches = srch.consecutive_batches(x, y, B)
+  for _ in range(steps):
+    plan.train_step(*next(batches))
+  bench.dump_outputs(plan, str(tmp_path))
+  last = plan.last_losses()
+  labels = y[(steps - 1) * B:steps * B]
+  for k, c in enumerate(plan.candidates):
+    def load(key):
+      a = np.load(str(tmp_path / ("%s.%s.npy" % (c.spec.name, key))))
+      assert a.dtype in (np.float32, np.float64)
+      return a
+    for key, want in c.state_dict().items():
+      if key != "trace":
+        np.testing.assert_array_equal(load(key), want)
+    np.testing.assert_array_equal(load("losses"), last[k])
+    logits = load("logits").astype(np.float64)
+    assert logits.shape == (B, C)
+    z = logits - logits.max(axis=1, keepdims=True)
+    xent = np.mean(np.log(np.exp(z).sum(axis=1)) - z[np.arange(B), labels])
+    assert abs(xent - last[k][0]) < 1e-5
+
+
+@pytest.mark.gpu
 def test_config5_sweep_at_real_widths(built_lib):
   """BASELINE configs[4] at its real size for one iteration: 32 candidates, depth 1..8 x width {128,256,512,1024},
   B=4096 (241 MFLOP per example summed over the candidates), 3 steps against the oracle."""
