@@ -29,9 +29,6 @@
 namespace adn {
 
 namespace convtc {
-bool bwd_supported(int h, int w, int cin, int f);
-int bwd(const float* images, const uint32_t* argmax, const float* dpooled, float* partials, int* n_partials, int64_t batch,
-        int h, int w, int cin, int f, cudaStream_t st);
 bool supported(int h, int w, int cin, int f);
 int fwd(const float* images, const float* kernel, const float* bias, void* out_planes, uint32_t* argmax, int64_t batch,
         int h, int w, int cin, int f, cudaStream_t st);
@@ -43,13 +40,6 @@ namespace conv {
 static bool use_tc() {      // read per call (host side, cheap): tests switch it at run time
   const char* e = getenv("ADN_CONV_PATH");
   return !(e && (e[0] == 's' || e[0] == 'S'));
-}
-
-// The tcgen05 backward (conv_stem_tc.cu) is correct but, with its serial build -> MMA -> drain per warpgroup, slower
-// than the SIMT gather (204 vs 136 us at B=4096, profiles/r1h_conv_tc_*.txt): opt-in with ADN_CONV_BWD_PATH=tcgen05.
-static bool use_tc_bwd() {
-  const char* e = getenv("ADN_CONV_BWD_PATH");
-  return e && (e[0] == 't' || e[0] == 'T');
 }
 
 static constexpr int FWD_THREADS = 256;
@@ -362,17 +352,6 @@ extern "C" int adn_conv_stem_bwd(const float* images, const uint32_t* argmax, co
   if (!workspace || workspace_bytes < need)
     return fail(ADN_ERR_WORKSPACE, "adn_conv_stem_bwd: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)need);
   const int kf = 9 * channels * filters;
-  if (conv::use_tc_bwd() && convtc::bwd_supported(height, width, channels, filters)) {
-    int n_part = 0;
-    if (int rc = convtc::bwd(images, argmax, dpooled, static_cast<float*>(workspace), &n_part, batch, height, width, channels,
-                             filters, as_stream(stream)))
-      return rc;
-    const int n_out = kf + filters;
-    conv::conv_stem_reduce_kernel<<<(n_out * 32 + 255) / 256, 256, 0, as_stream(stream)>>>(static_cast<float*>(workspace), n_part,
-                                                                                     n_out, kf, dkernel, dbias);
-    ADN_CHECK_LAUNCH("conv_stem_reduce");
-    return ADN_OK;
-  }
   // G thread groups of channels*filters threads share the pooled pixels of an image (even, so threads % 32 == 0)
   int groups = (384 / (channels * filters)) & ~1;
   groups = groups < 2 ? 2 : (groups > 16 ? 16 : groups);

@@ -13,19 +13,19 @@
 //
 // fp32 accuracy: 3xTF32 (a_hi b_hi + a_lo b_hi + a_hi b_lo), K <= 48, one TMEM accumulator.
 //
-// Per CTA (256 threads = 2 warpgroups, 1 CTA per SM): the image is staged zero-padded in shared memory with
-// cp.async (double buffered); each warpgroup takes a tile of 128 pooled pixels: every thread gathers its own A row
-// from the staged image (LDS.64), splits it and writes hi / lo in the canonical K-major SWIZZLE_128B layout
-// (16-byte chunk index XOR row%8 -- what TMA would have produced), fence.proxy.async, one elected thread issues
-// the MMAs and commits to the warpgroup's mbarrier, then all 128 threads read their accumulator row with
-// tcgen05.ld (warp w reads TMEM lanes 32(w%4)..) and run the epilogue.  W' (hi / lo, K-major) is built once per CTA.
+// Per CTA (512 threads = 4 warpgroups, 1 CTA per SM, images grid-strided): the image is staged zero-padded in shared
+// memory with cp.async (a ring of 2 or 4 images).  Two builder warpgroups each take a tile of 128 pooled pixels: every
+// thread gathers its own A row from the staged image (LDS.64), splits it and writes hi / lo in the canonical K-major
+// SWIZZLE_128B layout (16-byte chunk index XOR row%8 -- what TMA would have produced), fence.proxy.async, one elected
+// thread issues the MMAs and commits to the accumulator's mbarrier.  Two epilogue warpgroups read their accumulator
+// rows with tcgen05.ld (warp w reads TMEM lanes 32(w%4)..) and run the epilogue while the builders fill the next
+// tile.  W' (hi / lo, K-major) is built once per CTA.  The backward is the SIMT kernel in conv_stem.cu.
 #include "common.cuh"
 #include "plane_fmt.cuh"
 
 namespace adn {
 namespace convtc {
 
-static constexpr int THREADS = 256;
 static constexpr int TILE_BYTES = 128 * 128;   // one k-block (32 floats) of a 128-row K-major SWIZZLE_128B tile
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -96,24 +96,13 @@ __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&r)[16]) {
-  uint32_t u[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7]),
-        "=r"(u[8]), "=r"(u[9]), "=r"(u[10]), "=r"(u[11]), "=r"(u[12]), "=r"(u[13]), "=r"(u[14]), "=r"(u[15])
-      : "r"(taddr));
-#pragma unroll
-  for (int i = 0; i < 16; ++i) r[i] = __uint_as_float(u[i]);
-}
 // byte offset of element (row, k) inside one k-block tile ([rows][32 floats], SWIZZLE_128B)
 __device__ __forceinline__ uint32_t sw128(int row, int k) {
   return (uint32_t)((row >> 3) * 1024 + (row & 7) * 128 + ((((k >> 2) ^ (row & 7)) & 7) << 4) + ((k & 3) << 2));
 }
 
 template <int CIN>
-__device__ __forceinline__ void stage_image(float* s_img, const float* img, int H, int W, int tid, int nthreads = THREADS) {
+__device__ __forceinline__ void stage_image(float* s_img, const float* img, int H, int W, int tid, int nthreads) {
   const int row = W * CIN;
   const int prow = (W + 2) * CIN;
   const int lane = tid & 31;
@@ -352,264 +341,6 @@ conv_stem_tc_fwd_kernel(const float* __restrict__ images, const float* __restric
   }
 }
 
-// ---------------------------------------------------------------------------------------------------------------
-// Backward of the stem on tcgen05: with G'[p][(pos, f)] = g[p][f] * [argmax(p, f) == pos] (the pooled-feature
-// gradient routed to its arg-max position) the kernel gradient of the expanded weights is
-//     dW'[(pos, f)][k] = sum_p G'[p][(pos, f)] * A[p][k]
-// -- a GEMM whose reduction runs over pooled pixels, so both operands are staged TRANSPOSED (K-major in the pooled
-// index): M side = G'^T [4F rows (128 with zero rows)][64 px], N side = A^T [K rows][64 px], 3xTF32, 24 MMAs
-// (M128 N=K K8) per tile of 64 pooled pixels.  A warpgroup's 128 threads split a tile: threads 0-63 build A^T from the
-// staged image and later drain the accumulator, threads 64-127 fetch g / arg-max from global memory and build G'^T.
-// Two-level accumulation: TMEM holds one tile's sum, the drainers add it (RN) into registers; at the end
-// dK[ky,kx,c,f] = sum_pos dW'[(pos,f)][(ky+dy, kx+dx, c)] is folded in fixed order and written as this CTA's partial
-// (same format as the SIMT backward, reduced by conv_stem_reduce_kernel).
-template <int CIN, int F>
-__global__ void __launch_bounds__(THREADS, 1)
-conv_stem_tc_bwd_kernel(const float* __restrict__ images, const uint32_t* __restrict__ argmax,
-                        const float* __restrict__ dpooled, float* __restrict__ partials, int64_t B, int H, int W) {
-  constexpr int K = 16 * CIN;              // patch size = GEMM N
-  static_assert(4 * F <= 64, "(pos, f) rows must fit TMEM lanes 0..63");
-  constexpr int PXT = 64;                  // pooled pixels per tile = GEMM K
-  constexpr int GB = 2 * TILE_BYTES;       // one plane of G'^T: 2 k-blocks of [128 rows][32 px]
-  constexpr int AB = 2 * K * 128;          // one plane of A^T : 2 k-blocks of [K rows][32 px]
-  constexpr int WGB = 2 * GB + 2 * AB;     // bytes per warpgroup
-  constexpr int TMEM_COLS = 128;           // two accumulators of K (<= 48) columns at column 0 and 64
-  constexpr int K9 = 9 * CIN;
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  const int pimg = (H + 2) * (W + 2) * CIN;
-  float* s_img0 = reinterpret_cast<float*>(base + 2 * WGB);
-  uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_img0 + 2 * pimg);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(s_bar + 2);
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int wg = tid >> 7, r = tid & 127;
-  const int half = r >> 6, q = r & 63;     // half 0: A^T builder + drainer (TMEM lanes 0..63), half 1: G'^T builder
-  uint8_t* g_hi = base + wg * WGB;
-  uint8_t* g_lo = g_hi + GB;
-  uint8_t* at_hi = g_lo + GB;
-  uint8_t* at_lo = at_hi + AB;
-  // zero everything once: rows MU..127 of G'^T stay zero for the whole kernel, image borders too
-  for (int i = tid; i < (2 * WGB) / 16; i += THREADS) reinterpret_cast<float4*>(base)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-  for (int i = tid; i < 2 * pimg; i += THREADS) s_img0[i] = 0.f;
-  if (warp == 0) {
-    if (lane == 0) {
-      mbar_init(smem_u32(&s_bar[0]), 1);
-      mbar_init(smem_u32(&s_bar[1]), 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"((uint32_t)TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  fence_async_smem();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tmem_acc = tmem_base + (uint32_t)(wg * 64);
-  const uint32_t tmem_row = tmem_acc + ((uint32_t)((warp & 3) * 32) << 16);
-  const uint32_t idesc = make_idesc(128, K);
-  const uint32_t g_addr = smem_u32(g_hi), at_addr = smem_u32(at_hi);
-  const uint32_t bar = smem_u32(&s_bar[wg]);
-  uint32_t phase = 0;
-
-  const int PH = H / 2, PW = W / 2, P = PH * PW;
-  const int tiles = (P + PXT - 1) / PXT;
-  const int prow = (W + 2) * CIN;
-  const int64_t img_elems = (int64_t)H * W * CIN;
-  const int64_t cols = (int64_t)P * F;
-  float acc[K];                            // drainers: dW'[(pos, f) = q][k] summed over this CTA's tiles
-#pragma unroll
-  for (int k = 0; k < K; ++k) acc[k] = 0.f;
-  float accb[F];                           // G builders: sum of g over their pooled pixels, per filter
-#pragma unroll
-  for (int f = 0; f < F; ++f) accb[f] = 0.f;
-
-  int64_t b = blockIdx.x;
-  int buf = 0;
-  if (b < B) stage_image<CIN>(s_img0, images + b * img_elems, H, W, tid);
-  cp_async_commit();
-  for (; b < B; b += gridDim.x, buf ^= 1) {
-    const int64_t nb = b + gridDim.x;
-    if (nb < B) stage_image<CIN>(s_img0 + (buf ^ 1) * pimg, images + nb * img_elems, H, W, tid);
-    cp_async_commit();
-    cp_async_wait<1>();
-    __syncthreads();
-    const float* s_img = s_img0 + buf * pimg;
-    for (int tile = wg; tile < tiles; tile += 2) {
-      const int p = tile * PXT + q;
-      const bool valid = p < P;
-      const uint32_t kblk = (uint32_t)(q >> 5);      // which 32-pixel k-block this pooled pixel falls in
-      const int col = q & 31;
-      if (half == 0) {
-        // ---- A^T: column `q` of every row k (the 4x4xCIN patch of pooled pixel p) ----
-        const int py = valid ? p / PW : 0, px = valid ? p - py * PW : 0;
-        const float* patch = s_img + (2 * py) * prow + (2 * px) * CIN;
-#pragma unroll
-        for (int c4 = 0; c4 < K / 4; ++c4) {
-          const int i = (CIN == 3) ? c4 / 3 : c4;
-          const int o = (CIN == 3) ? (c4 % 3) * 4 : 0;
-          float2 v0 = *reinterpret_cast<const float2*>(patch + i * prow + o);
-          float2 v1 = *reinterpret_cast<const float2*>(patch + i * prow + o + 2);
-          if (!valid) { v0 = make_float2(0.f, 0.f); v1 = v0; }
-          const float v[4] = {v0.x, v0.y, v1.x, v1.y};
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            const int k = c4 * 4 + e;
-            const float h = rna_tf32(v[e]);
-            const uint32_t off = kblk * (uint32_t)(K * 128) + sw128(k, col);
-            *reinterpret_cast<float*>(at_hi + off) = h;
-            *reinterpret_cast<float*>(at_lo + off) = rna_tf32(v[e] - h);
-          }
-        }
-      } else {
-        // ---- G'^T: column `q` of rows (pos, f): g at the arg-max position, zero at the other three ----
-#pragma unroll
-        for (int f0 = 0; f0 < F; f0 += 16) {
-          float g[16];
-          uint32_t aw = 0u;
-          if (valid) {
-            const float4* src = reinterpret_cast<const float4*>(dpooled + b * cols + (int64_t)p * F + f0);
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              const float4 t = __ldg(src + e);
-              g[4 * e] = t.x; g[4 * e + 1] = t.y; g[4 * e + 2] = t.z; g[4 * e + 3] = t.w;
-            }
-            aw = __ldg(argmax + b * (cols / 16) + ((int64_t)p * F + f0) / 16);
-          } else {
-#pragma unroll
-            for (int e = 0; e < 16; ++e) g[e] = 0.f;
-          }
-#pragma unroll
-          for (int e = 0; e < 16; ++e) {
-            const uint32_t pos = (aw >> (2 * e)) & 3u;
-            const float h = rna_tf32(g[e]);
-            const float l = rna_tf32(g[e] - h);
-            accb[f0 + e] += g[e];
-#pragma unroll
-            for (int s = 0; s < 4; ++s) {
-              const uint32_t off = kblk * (uint32_t)TILE_BYTES + sw128(s * F + f0 + e, col);
-              *reinterpret_cast<float*>(g_hi + off) = (pos == (uint32_t)s) ? h : 0.f;
-              *reinterpret_cast<float*>(g_lo + off) = (pos == (uint32_t)s) ? l : 0.f;
-            }
-          }
-        }
-      }
-      fence_async_smem();
-      tc_fence_before();
-      wg_barrier(wg);
-      if ((warp & 3) == 0) {
-        if (elect_one()) {
-          tc_fence_after();
-          uint32_t accum = 0;
-#pragma unroll
-          for (int prod = 0; prod < 3; ++prod) {       // g_hi a_hi, g_lo a_hi, g_hi a_lo
-            const uint32_t gg = g_addr + (prod == 1 ? GB : 0);
-            const uint32_t aa = at_addr + (prod == 2 ? AB : 0);
-#pragma unroll
-            for (int ks = 0; ks < PXT / 8; ++ks) {
-              const uint32_t da = desc_lo(gg + (ks >> 2) * TILE_BYTES + (ks & 3) * 32);
-              const uint32_t db = desc_lo(aa + (ks >> 2) * (K * 128) + (ks & 3) * 32);
-              umma_tf32(tmem_acc, da, db, idesc, accum);
-              accum = 1;
-            }
-          }
-          umma_commit(bar);
-        }
-        __syncwarp();
-      }
-      mbar_wait(bar, phase);
-      phase ^= 1;
-      tc_fence_after();
-      if (half == 0) {                      // warps 0-1 of the warpgroup own TMEM lanes 0..63 = rows (pos, f) < 64
-#pragma unroll
-        for (int c0 = 0; c0 < K; c0 += 16) {
-          float t[16];
-          tmem_ld16(tmem_row + (uint32_t)c0, t);
-          tmem_ld_wait();
-#pragma unroll
-          for (int e = 0; e < 16; ++e) acc[c0 + e] += t[e];
-        }
-      }
-      tc_fence_before();
-    }
-    __syncthreads();
-  }
-  // ---- fold: dump dW' and the bias sums to shared memory (the operand tiles are free now), then fixed-order sums ----
-  tc_fence_before();
-  __syncthreads();
-  float* s_d = reinterpret_cast<float*>(base);                  // [2 wg][64 rows][K]
-  float* s_db = s_d + 2 * 64 * K;                               // [2 wg][64 px][F]
-  if (half == 0) {
-#pragma unroll
-    for (int k = 0; k < K; ++k) s_d[(wg * 64 + q) * K + k] = acc[k];
-  } else {
-#pragma unroll
-    for (int f = 0; f < F; ++f) s_db[(wg * 64 + q) * F + f] = accb[f];
-  }
-  __syncthreads();
-  float* mine = partials + (size_t)blockIdx.x * (K9 * F + F);
-  for (int t = tid; t < K9 * F; t += THREADS) {
-    const int f = t % F, kc = t / F;                            // kc = (ky*3 + kx)*CIN + c
-    const int c = kc % CIN, kyx = kc / CIN, ky = kyx / 3, kx = kyx - ky * 3;
-    float sum = 0.f;
-    for (int w2 = 0; w2 < 2; ++w2)
-      for (int pos = 0; pos < 4; ++pos) {
-        const int n = pos * F + f;
-        if (n < 64) {
-          const int k = ((ky + (pos >> 1)) * 4 + (kx + (pos & 1))) * CIN + c;
-          sum += s_d[(w2 * 64 + n) * K + k];
-        }
-      }
-    mine[t] = sum;
-  }
-  for (int f = tid; f < F; f += THREADS) {
-    float sum = 0.f;
-    for (int i = 0; i < 2 * 64; ++i) sum += s_db[i * F + f];
-    mine[K9 * F + f] = sum;
-  }
-  __syncthreads();
-  if (warp == 0) {
-    __syncwarp();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TMEM_COLS)
-                 : "memory");
-  }
-}
-
-template <int CIN, int F>
-static size_t bwd_smem_bytes(int h, int w) {
-  constexpr int K = 16 * CIN;
-  return 1024 + (size_t)2 * (2 * 2 * TILE_BYTES + 2 * 2 * K * 128) + (size_t)2 * (h + 2) * (w + 2) * CIN * 4 + 2 * 8 + 16;
-}
-
-bool bwd_supported(int h, int w, int cin, int f) {
-  if (f != 16) return false;               // (pos, f) rows must fit TMEM lanes 0..63 of the drainer warps
-  const size_t smem = cin == 3 ? bwd_smem_bytes<3, 16>(h, w) : bwd_smem_bytes<1, 16>(h, w);
-  return smem <= 227 * 1024;
-}
-
-// writes `*n_partials` per-CTA partials [9*cin*f + f] into `partials`
-int bwd(const float* images, const uint32_t* argmax, const float* dpooled, float* partials, int* n_partials, int64_t batch,
-        int h, int w, int cin, int f, cudaStream_t st) {
-  const int64_t cap = sm_count();
-  const int grid = (int)(batch < cap ? batch : cap);
-  *n_partials = grid;
-  if (cin == 3) {
-    const size_t smem = bwd_smem_bytes<3, 16>(h, w);
-    auto kern = conv_stem_tc_bwd_kernel<3, 16>;
-    kern<<<grid, THREADS, smem, st>>>(images, argmax, dpooled, partials, batch, h, w);
-  } else {
-    const size_t smem = bwd_smem_bytes<1, 16>(h, w);
-    auto kern = conv_stem_tc_bwd_kernel<1, 16>;
-    kern<<<grid, THREADS, smem, st>>>(images, argmax, dpooled, partials, batch, h, w);
-  }
-  ADN_CHECK_LAUNCH("conv_stem_tc_bwd");
-  return ADN_OK;
-}
-
 template <int CIN, int F>
 static size_t smem_bytes(int h, int w) {
   constexpr int K = 16 * CIN, KB = (K + 31) / 32, N = 4 * F;
@@ -634,7 +365,6 @@ int init() {
 #define ADN_CONVTC_ATTR(K) ADN_CUDA(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024))
   ADN_CONVTC_ATTR((conv_stem_tc_fwd_kernel<1, 16>)); ADN_CONVTC_ATTR((conv_stem_tc_fwd_kernel<3, 16>));
   ADN_CONVTC_ATTR((conv_stem_tc_fwd_kernel<1, 32>)); ADN_CONVTC_ATTR((conv_stem_tc_fwd_kernel<3, 32>));
-  ADN_CONVTC_ATTR((conv_stem_tc_bwd_kernel<1, 16>)); ADN_CONVTC_ATTR((conv_stem_tc_bwd_kernel<3, 16>));
 #undef ADN_CONVTC_ATTR
   return ADN_OK;
 }

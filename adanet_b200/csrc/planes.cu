@@ -95,12 +95,11 @@ struct GemmParams {
   int M, N;
   int tiles_m, tiles_n, splits;
   int tiles;             // tiles_m * tiles_n
-  float inv_tiles, inv_tiles_n, inv_tiles_m;   // reciprocals for the division-free item decode (counts stay far below 2^21)
+  float inv_tiles, inv_tiles_n;   // reciprocals for the division-free item decode (counts stay far below 2^21)
   int total_kb;          // k-blocks over the whole K
   int kb_per_split;
   int a_mn, b_mn;        // operand majorness (0 = K-major box, 1 = MN-major box)
   int out_planes;        // 1: result written as split planes (out / out_lo / out_bits), 0: dense fp32
-  int m_fastest;         // work-item order: 1 = row blocks fastest (write locality), 0 = column blocks fastest (A reuse in L2)
   // output: dense row-major (ldc) / split-K partial [split][M][N], or planes
   void* out;             // dense base | hi plane base
   void* out_lo;          // lo plane base (OUT_PLANES)
@@ -253,7 +252,8 @@ __device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t (&r)[3
       : "r"(taddr));
 }
 
-// work item -> (tile_m, tile_n, split).  n fastest so concurrently resident CTAs share A tiles.
+// work item -> (tile_m, tile_n, split).  n fastest so concurrently resident CTAs share A tiles through L2 (A is the
+// big operand of the long-K layers).
 struct Item {
   int m0, n0, kb0, nkb, split;
 };
@@ -266,15 +266,9 @@ __device__ __forceinline__ Item decode_item(const GemmParams& g, int item) {
   Item it;
   it.split = (g.splits == 1) ? 0 : fast_div(item, g.inv_tiles);
   const int t = item - it.split * g.tiles;
-  if (g.m_fastest) {            // consecutive items = consecutive row blocks of the same column block
-    const int tn = fast_div(t, g.inv_tiles_m);
-    it.n0 = tn * BN;
-    it.m0 = (t - tn * g.tiles_m) * BM;
-  } else {
-    const int tm = (g.tiles_n == 1) ? t : fast_div(t, g.inv_tiles_n);
-    it.m0 = tm * BM;
-    it.n0 = (t - tm * g.tiles_n) * BN;
-  }
+  const int tm = (g.tiles_n == 1) ? t : fast_div(t, g.inv_tiles_n);
+  it.m0 = tm * BM;
+  it.n0 = (t - tm * g.tiles_n) * BN;
   it.kb0 = it.split * g.kb_per_split;
   it.nkb = min(g.total_kb, it.kb0 + g.kb_per_split) - it.kb0;
   return it;
@@ -294,8 +288,8 @@ __device__ __forceinline__ void st_global_v8(void* p, const uint32_t (&w)[8]) {
                : "memory");
 }
 
-// split 32 values of one row into the two planes and write them with 256-bit stores (TF32 planes, and fp16 planes
-// under ADN_PL_TMA_STORE=0; the default fp16 path is store_slice_tma_hi / _lo below)
+// split 32 values of one row into the two planes and write them with 256-bit stores (TF32 planes, and fp16 planes whose
+// buffers are not 128 B aligned or hold an odd number of 32-column blocks; other fp16 planes take store_slice_tma_hi / _lo)
 template <int FMT>
 __device__ __forceinline__ void store_row32_planes(const GemmParams& g, const float* a, int my_row, int cbase) {
   constexpr int BK = Fmt<FMT>::BK;
@@ -478,7 +472,7 @@ __device__ __forceinline__ void emit_slice(const GemmParams& g, const bool OUT_P
     emit_slice_fwd_planes<FMT>(g, a, lane, mrow0, cbase, o_hi, o_lo, smem_u32(stage));
     return;
   }
-  if (EPI == EPI_MASK && OUT_PLANES && bias_in_acc) {      // (the single-CTA kernel's direct path; out_mul is 1 for planes)
+  if (EPI == EPI_MASK && OUT_PLANES && bias_in_acc) {
     emit_slice_mask_planes<FMT>(g, a, mwq, lane, mrow0, cbase, o_hi, o_lo, smem_u32(stage));
     return;
   }
@@ -872,363 +866,6 @@ pl_gemm_kernel(const __grid_constant__ Group grp) {
 }
 
 // ---------------------------------------------------------------------------------
-// CTA-pair GEMM kernel (tcgen05 cta_group::2): one 256 x 256 tile per pair of SMs, grouped like pl_gemm_kernel.
-//
-// With fp16 planes the tensor pipe retires a 128 B k-block of the 128x128 single-CTA tile in 768 clk while that
-// tile needs 64 KiB of operands for it: 85 B/clk per SM out of L2 (21 TB/s chip-wide at the cuBLAS fp16 rate) and
-// a 3-stage ring that covers only ~0.9 us of TMA latency -- profiles/r2e_gemm_single_ncu_full.txt shows the
-// tensor pipe 55-59 % active with nothing else saturated.  The pair tile moves (128 A rows + 128 B rows) per SM for
-// twice the tensor work: half the L2 and shared-memory traffic per flop, twice the latency cover per stage.
-//   CTA rank r of the pair owns A rows / D rows [m0 + 128 r, +128) and supplies B rows
-//   [n0 + r n_inst/2, + n_inst/2); the leader (rank 0) issues tcgen05.mma.cta_group::2 (M = 256,
-//   N = n_inst <= 256, trimmed to the live columns) for both SMs.
-//   TMEM per SM (512 columns): H [0,256) = hi*hi partial sums of ONE 128-K chunk, S [256,512) = cross
-//   terms of the whole tile.  H is single-buffered: the next chunk starts with its cross-term MMAs
-//   while the epilogue warps of both CTAs drain H into registers.
-//   Barriers: TMA of both CTAs -> leader's full[s] (tx bytes of both); commit multicast -> both CTAs'
-//   empty[s] / acc_full; epilogue warps of both CTAs -> leader's acc_empty / s_empty (remote arrive).
-// ---------------------------------------------------------------------------------
-static constexpr int BM2 = 256, BN2 = 256;
-static constexpr int EPI_WARPS2 = 16;              // 4 TMEM lane quadrants x 4 column groups of 64: the single-buffered H must be
-static constexpr int NUM_THREADS2 = 64 + 32 * EPI_WARPS2;   // drained inside the cross-term window of the next chunk (1024 clk)
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t mapa_rank(uint32_t smem_addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// Remote arrive on the leader's barrier.  Default semantics (release at CTA scope), as CUTLASS's ClusterBarrier does: what
-// these barriers hand over is TMEM state, ordered by the tcgen05 fences around them -- no generic-proxy data.  A
-// `.release.cluster` arrive instead waits for every global store the warp has in flight (the previous tile's 64 KB of
-// plane stores) and was 30 % of the kernel's stall samples (profiles/r2k_pair_kernel_ncu.txt).
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// wait on a local barrier whose arrivals come from other CTAs of the cluster: the plain (CTA-scope acquire) wait; the
-// cluster-scope acquire form compiles to an L1 invalidation (CCTL.IVALL) per successful wait
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) { mbar_wait(bar, parity); }
-__device__ __forceinline__ void tma_load_3d_2sm(const CUtensorMap* map, uint32_t bar_cluster, uint32_t dst, int c0, int c1,
-                                                int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_cluster), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-template <int FMT>
-__device__ __forceinline__ void umma_2sm(uint32_t tmem_d, uint32_t da_lo, uint32_t db_lo, uint32_t da_hi, uint32_t db_hi,
-                                         uint32_t idesc, uint32_t accum) {
-  if (FMT == FMT_F16) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %3};\n\t"
-        "mov.b64 db, {%2, %4};\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}"
-        ::"r"(tmem_d), "r"(da_lo), "r"(db_lo), "r"(da_hi), "r"(db_hi), "r"(idesc), "r"(accum)
-        : "memory");
-  } else {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %3};\n\t"
-        "mov.b64 db, {%2, %4};\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::tf32 [%0], da, db, %5, p;\n\t}"
-        ::"r"(tmem_d), "r"(da_lo), "r"(db_lo), "r"(da_hi), "r"(db_hi), "r"(idesc), "r"(accum)
-        : "memory");
-  }
-}
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {   // arrives on the barrier at this offset in BOTH CTAs
-  asm volatile(
-      "{\n\t.reg .b16 m;\n\tmov.b16 m, 3;\n\t"
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], m;\n\t}"
-      ::"r"(bar)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-
-struct Item2 {
-  int m0, n0, kb0, nkb, split, n_inst;
-};
-template <int FMT>
-__device__ __forceinline__ Item2 decode_item2(const GemmParams& g, int item) {
-  Item2 it;
-  it.split = (g.splits == 1) ? 0 : fast_div(item, g.inv_tiles);      // 256 x 256 tiles
-  const int t = item - it.split * g.tiles;
-  const int tm = (g.tiles_n == 1) ? t : fast_div(t, g.inv_tiles_n);
-  it.m0 = tm * BM2;
-  it.n0 = (t - tm * g.tiles_n) * BN2;
-  it.kb0 = it.split * g.kb_per_split;
-  it.nkb = min(g.total_kb, it.kb0 + g.kb_per_split) - it.kb0;
-  // live columns in steps of 2 k-block widths: each CTA's half must start on a k-block boundary of an MN-major B
-  constexpr int GR = 2 * Fmt<FMT>::BK;
-  it.n_inst = min(BN2, ((g.N - it.n0 + GR - 1) / GR) * GR);
-  return it;
-}
-
-template <int FMT, int EPI>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS2, 1)
-pl_gemm2_kernel(const __grid_constant__ Group grp) {
-  constexpr int BK = Fmt<FMT>::BK;
-  constexpr int CHUNK = Fmt<FMT>::CHUNK;
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = smem_raw;
-  if ((smem_u32(smem) & 1023u) != 0u) __trap();
-  float* epi_stage = reinterpret_cast<float*>(smem + STAGES * STAGE_BYTES);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + STAGES * STAGE_BYTES + EPI_BYTES);
-  uint64_t* full_bar = bars;                       // [STAGES]  leader's: TMA of both CTAs -> MMA
-  uint64_t* empty_bar = bars + STAGES;             // [STAGES]  each CTA's: MMA commit (multicast) -> TMA
-  uint64_t* acc_full = bars + 2 * STAGES;          // [1]       each CTA's: MMA commit (multicast) -> epilogue
-  uint64_t* acc_empty = bars + 2 * STAGES + 1;     // [1]       leader's: epilogue warps of both CTAs -> MMA (H drained)
-  uint64_t* s_empty = bars + 2 * STAGES + 2;       // [1]       leader's: epilogue warps of both CTAs -> MMA (S drained)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 3);
-
-  const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
-  const int lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
-  const int n_items = grp.total_items;
-
-  if (warp == 0 && lane < grp.n) {
-    tma_prefetch_desc(&grp.p[lane].a_hi);
-    tma_prefetch_desc(&grp.p[lane].a_lo);
-    tma_prefetch_desc(&grp.p[lane].b_hi);
-    tma_prefetch_desc(&grp.p[lane].b_lo);
-  }
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < STAGES; ++s) {
-        mbar_init(smem_u32(&full_bar[s]), 1);
-        mbar_init(smem_u32(&empty_bar[s]), 1);
-      }
-      mbar_init(smem_u32(acc_full), 1);
-      mbar_init(smem_u32(acc_empty), 2 * EPI_WARPS2);
-      mbar_init(smem_u32(s_empty), 2 * EPI_WARPS2);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"((uint32_t)TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();          // both CTAs' barriers are initialised before any remote arrive / multicast commit
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ================= TMA producer (both CTAs: own A rows, own half of B) =================
-    if (lane == 0) {
-      uint32_t s = 0, ph = 0;
-      int cur = 0, next0 = first_next0(grp);
-      const uint32_t smem0 = smem_u32(smem);
-      for (int item = pair; item < n_items; item += npairs) {
-        cur = find_problem(grp, cur, item, next0);
-        const Problem& pr = grp.p[cur];
-        const GemmParams& g = pr.g;
-        const Item2 it = decode_item2<FMT>(g, item - pr.item0);
-        const int a_row = it.m0 + (int)rank * 128;
-        const int b_row = it.n0 + (int)rank * (it.n_inst >> 1);
-        for (int kb = 0; kb < it.nkb; ++kb) {
-          mbar_wait(smem_u32(&empty_bar[s]), ph ^ 1);
-          if (rank == 0) mbar_expect_tx(smem_u32(&full_bar[s]), 2 * STAGE_BYTES);   // bytes of both CTAs
-          const uint32_t fb = mapa_rank(smem_u32(&full_bar[s]), 0);                 // leader's barrier
-          const uint32_t base = smem0 + s * STAGE_BYTES;
-          const int kc = it.kb0 + kb;
-          const int a1 = g.a_mn ? kc * BK : a_row, a2 = g.a_mn ? (a_row / BK) : kc;
-          const int b1 = g.b_mn ? kc * BK : b_row, b2 = g.b_mn ? (b_row / BK) : kc;
-          tma_load_3d_2sm(&pr.a_hi, fb, base + 0 * TILE_BYTES, 0, a1, a2);
-          tma_load_3d_2sm(&pr.a_lo, fb, base + 1 * TILE_BYTES, 0, a1, a2);
-          tma_load_3d_2sm(&pr.b_hi, fb, base + 2 * TILE_BYTES, 0, b1, b2);
-          tma_load_3d_2sm(&pr.b_lo, fb, base + 3 * TILE_BYTES, 0, b1, b2);
-          if (++s == STAGES) { s = 0; ph ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ================= MMA issuer (leader CTA only) =================
-    if (rank == 0) {
-      const uint32_t smem0 = smem_u32(smem);
-      const uint32_t acc_h = tmem_base, acc_s = tmem_base + 256;
-      uint32_t s = 0, ph = 0, gchunk = 0, tile_i = 0;
-      int cur = 0, next0 = first_next0(grp);
-      for (int item = pair; item < n_items; item += npairs, ++tile_i) {
-        cur = find_problem(grp, cur, item, next0);
-        const GemmParams& g = grp.p[cur].g;
-        const Item2 it = decode_item2<FMT>(g, item - grp.p[cur].item0);
-        const uint32_t dah = desc_hi_word<FMT>(g.a_mn), dbh = desc_hi_word<FMT>(g.b_mn);
-        const uint32_t a_lo0 = desc_lo_word<FMT>(smem0, g.a_mn);
-        const uint32_t b_lo0 = desc_lo_word<FMT>(smem0 + 2 * TILE_BYTES, g.b_mn);
-        const uint32_t a_step = g.a_mn ? Fmt<FMT>::MN_STEP : (32u >> 4);
-        const uint32_t b_step = g.b_mn ? Fmt<FMT>::MN_STEP : (32u >> 4);
-        const uint32_t idesc = make_idesc<FMT>(BM2, it.n_inst, g.a_mn, g.b_mn);
-        mbar_wait_cluster(smem_u32(s_empty), (tile_i & 1) ^ 1);     // cross-term accumulator drained by both CTAs
-        tc_fence_after();
-        uint32_t s_accum = 0;
-        for (int kb = 0; kb < it.nkb; kb += CHUNK, ++gchunk) {
-          const int nk = min(CHUNK, it.nkb - kb);
-          for (int kk = 0; kk < nk; ++kk) {
-            mbar_wait(smem_u32(&full_bar[s]), ph);
-            tc_fence_after();
-            const uint32_t so = s * (STAGE_BYTES >> 4);
-            if (kk == 0) {
-              // new chunk: cross terms first, so the tensor pipe stays busy while H is being drained
-              if (elect_one()) {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  const uint32_t a_hi = a_lo0 + so + k * a_step, a_lo = a_hi + (TILE_BYTES >> 4);
-                  const uint32_t b_hi = b_lo0 + so + k * b_step, b_lo = b_hi + (TILE_BYTES >> 4);
-                  umma_2sm<FMT>(acc_s, a_lo, b_hi, dah, dbh, idesc, (k == 0) ? s_accum : 1u);
-                  umma_2sm<FMT>(acc_s, a_hi, b_lo, dah, dbh, idesc, 1u);
-                }
-              }
-              __syncwarp();
-              mbar_wait_cluster(smem_u32(acc_empty), (gchunk & 1) ^ 1);   // H drained by both CTAs
-              tc_fence_after();
-              if (elect_one()) {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  const uint32_t a_hi = a_lo0 + so + k * a_step;
-                  const uint32_t b_hi = b_lo0 + so + k * b_step;
-                  umma_2sm<FMT>(acc_h, a_hi, b_hi, dah, dbh, idesc, (k == 0) ? 0u : 1u);
-                }
-                umma_commit_2sm(smem_u32(&empty_bar[s]));
-                if (nk == 1) umma_commit_2sm(smem_u32(acc_full));
-              }
-            } else {
-              if (elect_one()) {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  const uint32_t a_hi = a_lo0 + so + k * a_step, a_lo = a_hi + (TILE_BYTES >> 4);
-                  const uint32_t b_hi = b_lo0 + so + k * b_step, b_lo = b_hi + (TILE_BYTES >> 4);
-                  umma_2sm<FMT>(acc_s, a_lo, b_hi, dah, dbh, idesc, 1u);
-                  umma_2sm<FMT>(acc_s, a_hi, b_lo, dah, dbh, idesc, 1u);
-                  umma_2sm<FMT>(acc_h, a_hi, b_hi, dah, dbh, idesc, 1u);
-                }
-                umma_commit_2sm(smem_u32(&empty_bar[s]));
-                if (kk == nk - 1) umma_commit_2sm(smem_u32(acc_full));
-              }
-            }
-            __syncwarp();
-            s_accum = 1u;
-            if (++s == STAGES) { s = 0; ph ^= 1; }
-          }
-        }
-      }
-    }
-  } else {
-    // ================= epilogue warps 2..17 (both CTAs; 32 rows x 64 columns each) =================
-    const int quad = warp & 3;
-    const int cgrp = (warp - 2) >> 2;                // which 64 of the tile's 256 columns
-    const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
-    const uint32_t col_base = (uint32_t)(cgrp * 64);
-    float* stage = epi_stage + (warp - 2) * EPI_STAGE_FLOATS;
-    const uint32_t acc_empty_leader = mapa_rank(smem_u32(acc_empty), 0);
-    const uint32_t s_empty_leader = mapa_rank(smem_u32(s_empty), 0);
-    uint32_t gchunk = 0;
-    int cur = 0, next0 = first_next0(grp);
-    for (int item = pair; item < n_items; item += npairs) {
-      cur = find_problem(grp, cur, item, next0);
-      const GemmParams& g = grp.p[cur].g;
-      const Item2 it = decode_item2<FMT>(g, item - grp.p[cur].item0);
-      const int mrow0 = it.m0 + (int)rank * 128 + quad * 32;
-      const int ncol0 = it.n0 + (int)col_base;
-      const int my_row = mrow0 + lane;
-      const bool cols_live = (int)col_base < it.n_inst;   // warp-uniform: does this warp own any computed column?
-      uint32_t mw[2] = {0xffffffffu, 0xffffffffu};
-      if (EPI == EPI_MASK && g.mask_bits) {
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-          const int kbo = (ncol0 >> 5) + q;
-          mw[q] = (my_row < g.M && kbo < g.out_nb32) ? __ldg(g.mask_bits + (size_t)kbo * g.M + my_row) : 0u;
-        }
-      }
-      float acc[64];
-#pragma unroll
-      for (int j = 0; j < 64; ++j) acc[j] = 0.f;
-      const int nchunks = (it.nkb + CHUNK - 1) / CHUNK;
-      for (int c = 0; c < nchunks; ++c, ++gchunk) {
-        mbar_wait(smem_u32(acc_full), gchunk & 1);
-        tc_fence_after();
-        if (cols_live) {
-#pragma unroll
-          for (int t = 0; t < 2; ++t) {
-            uint32_t r0[32];
-            tmem_ld32_nowait(tmem_base + lane_base + col_base + t * 32, r0);
-            tmem_ld_wait();
-#pragma unroll
-            for (int j = 0; j < 32; ++j) acc[t * 32 + j] += __uint_as_float(r0[j]);   // fp32 RN adds
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(acc_empty_leader);      // H may be overwritten: the next chunk's hi*hi MMAs
-        if (c == nchunks - 1) {
-          if (cols_live) {
-#pragma unroll
-            for (int t = 0; t < 2; ++t) {
-              uint32_t r0[32];
-              tmem_ld32_nowait(tmem_base + lane_base + 256 + col_base + t * 32, r0);
-              tmem_ld_wait();
-#pragma unroll
-              for (int j = 0; j < 32; ++j) {
-                if (FMT == FMT_F16) acc[t * 32 + j] = fmaf(__uint_as_float(r0[j]), 1.0f / 2048.0f, acc[t * 32 + j]);
-                else acc[t * 32 + j] += __uint_as_float(r0[j]);
-              }
-            }
-          }
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive_cluster(s_empty_leader);
-        }
-      }
-      if (cols_live) {
-        float* dense = reinterpret_cast<float*>(g.out);
-        if (EPI == EPI_PARTIAL) dense += (size_t)it.split * g.M * g.N;
-        const bool out_planes = g.out_planes != 0;
-        const bool dense_vec = !out_planes && ((g.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(dense) & 15) == 0);
-        const int rows_ok = min(32, g.M - mrow0);
-#pragma unroll
-        for (int q = 0; q < 2; ++q)
-          if ((int)col_base + q * 32 < it.n_inst) {
-            if (EPI == EPI_BIAS_ACT && g.bias) {       // the direct epilogues expect the bias inside the accumulators
-              const int cb = ncol0 + q * 32;
-#pragma unroll
-              for (int j = 0; j < 32; ++j) acc[q * 32 + j] += (cb + j < g.N) ? __ldg(g.bias + cb + j) : 0.f;
-            }
-            emit_slice<FMT, EPI>(g, out_planes, &acc[q * 32], mw[q], stage, lane, mrow0, ncol0 + q * 32, rows_ok, dense,
-                                 dense_vec, true);
-          }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();          // neither CTA frees TMEM / exits while the peer may still use its smem or barriers
-  if (warp == 1) {
-    __syncwarp();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TMEM_COLS)
-                 : "memory");
-  }
-}
-
-// ---------------------------------------------------------------------------------
 // dense <-> planes conversion (inputs x / labels-side gradients / weights; everything
 // between two GEMMs is written as planes by the producing epilogue instead)
 // ---------------------------------------------------------------------------------
@@ -1364,11 +1001,6 @@ int init() {
     ADN_PL_ATTR(FMT_TF32, EPI_BIAS_ACT); ADN_PL_ATTR(FMT_TF32, EPI_MASK); ADN_PL_ATTR(FMT_TF32, EPI_PARTIAL);
     ADN_PL_ATTR(FMT_F16, EPI_BIAS_ACT); ADN_PL_ATTR(FMT_F16, EPI_MASK); ADN_PL_ATTR(FMT_F16, EPI_PARTIAL);
 #undef ADN_PL_ATTR
-#define ADN_PL_ATTR2(F, E) \
-  ok = ok && (cudaFuncSetAttribute(pl_gemm2_kernel<F, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) == cudaSuccess)
-    ADN_PL_ATTR2(FMT_TF32, EPI_BIAS_ACT); ADN_PL_ATTR2(FMT_TF32, EPI_MASK); ADN_PL_ATTR2(FMT_TF32, EPI_PARTIAL);
-    ADN_PL_ATTR2(FMT_F16, EPI_BIAS_ACT); ADN_PL_ATTR2(FMT_F16, EPI_MASK); ADN_PL_ATTR2(FMT_F16, EPI_PARTIAL);
-#undef ADN_PL_ATTR2
     if (!ok) {
       (void)cudaGetLastError();
       rc = fail(ADN_ERR_CUDA, "pl::init: cudaFuncSetAttribute(smem=%d) failed", SMEM_BYTES);
@@ -1480,10 +1112,6 @@ static int make_store_map(CUtensorMap* map, const void* plane, int64_t rows, int
   g_maps.emplace(key, *map);
   return ADN_OK;
 }
-static int store_mode() {      // ADN_PL_TMA_STORE=0: keep the direct 256-bit stores (A/B switch for profiles)
-  static const int env = getenv("ADN_PL_TMA_STORE") ? atoi(getenv("ADN_PL_TMA_STORE")) : 1;
-  return env;
-}
 
 // one GEMM of a group: operands + epilogue description (tiles / item numbering are filled at launch)
 struct GemmDesc {
@@ -1504,104 +1132,51 @@ static int encode_maps(int fmt, const GemmDesc& d, CUtensorMap* a_hi, CUtensorMa
   return ADN_OK;
 }
 
-// Work-item order of one problem.  Column blocks fastest lets the CTAs that run together share the A tile through
-// L2 (A is the big operand of the long-K layers); row blocks fastest makes them write adjacent 16 KB runs of the
-// same output k-block slab.  ADN_PL_MFAST: -1 heuristic (default), 0 / 1 force.
-static int item_order_m_fastest(const GemmParams& g) {
-  static const int env = getenv("ADN_PL_MFAST") ? atoi(getenv("ADN_PL_MFAST")) : -1;
-  if (env >= 0) return env;
-  (void)g;
-  return 0;
-}
-
 template <int FMT, int EPI>
 static void launch_kernel(const Group& grp, int grid, cudaStream_t st) {
   pl_gemm_kernel<FMT, EPI><<<grid, NUM_THREADS, SMEM_BYTES, st>>>(grp);
 }
-template <int FMT, int EPI>
-static void launch_kernel2(const Group& grp, int grid, cudaStream_t st) {
-  pl_gemm2_kernel<FMT, EPI><<<grid, NUM_THREADS2, SMEM_BYTES, st>>>(grp);
-}
 
-// Which GEMMs take the CTA-pair kernel.  ADN_PL_PAIR: 1 every GEMM, 2 the big ones (M, N >= 256, K >= 4 k-blocks),
-// unset / 0 none.  Measured on B200 (profiles/r2f_pair_vs_single_f16.txt): [32768,1024]x[1024,1024] fp16 planes
-// 206 us on pairs against 177 us on single CTAs (TF32 planes, round 1: equal), so the single-CTA kernel stays the
-// default and the pair kernel is kept as a tested alternative (tests force it through ADN_PL_PAIR=1).
-static int pair_mode() {
-  static const int env = getenv("ADN_PL_PAIR") ? atoi(getenv("ADN_PL_PAIR")) : 0;
-  return env;
-}
-static bool use_pair_shape(int fmt, int64_t M, int64_t N, int64_t total_kb, bool split_k = true) {
-  (void)fmt;
-  const int env = pair_mode();
-  if (env == 1) return true;
-  if (env == 2) return M >= 256 && N >= 256 && total_kb >= 4;
-  if (env == 3) return split_k && M >= 256 && N >= 256 && total_kb >= 4;     // the big dW GEMMs only
-  return false;
-}
-static bool use_pair(int fmt, const GemmDesc& d) {
-  // dropout lives in the single-CTA kernel's direct epilogue; mode 3 takes the split-K (dW) problems only
-  return d.g.drop_thresh == 0u && use_pair_shape(fmt, d.g.M, d.g.N, d.g.total_kb, d.g.out_planes == 0 && d.g.bias == nullptr &&
-                                                                                      d.g.mask_bits == nullptr && d.g.colsum_part == nullptr &&
-                                                                                      d.g.act == 0 && d.g.ldc == d.g.N && d.g.total_kb >= 64);
-}
-
-// n independent GEMMs of the same epilogue kind -> persistent launches of up to MAX_GROUP problems each; the problems
-// that take the CTA-pair kernel are launched as their own group(s)
+// n independent GEMMs of the same epilogue kind -> persistent launches of up to MAX_GROUP problems each
 template <int EPI>
 static int launch_group(int fmt, const GemmDesc* d, int n, cudaStream_t st, const char* what) {
-  for (int pass = 0; pass < 2; ++pass) {
-    const bool pair = pass == 0;
-    std::vector<int> idx;
-    for (int i = 0; i < n; ++i)
-      if (use_pair(fmt, d[i]) == pair) idx.push_back(i);
-    const int tm = pair ? BM2 : BM, tn = pair ? BN2 : BN;
-    for (size_t i0 = 0; i0 < idx.size(); i0 += MAX_GROUP) {
-      const int m = (int)std::min<size_t>(MAX_GROUP, idx.size() - i0);
-      Group grp;
-      memset(&grp, 0, sizeof(grp));
-      int items = 0;
-      for (int i = 0; i < m; ++i) {
-        const GemmDesc& src = d[idx[i0 + (size_t)i]];
-        Problem& pr = grp.p[i];
-        int rc = encode_maps(fmt, src, &pr.a_hi, &pr.a_lo, &pr.b_hi, &pr.b_lo, what);
-        if (rc) return rc;
-        pr.g = src.g;
-        pr.g.out_tma = 0;
-        if (!pair && fmt == FMT_F16 && EPI != EPI_PARTIAL && src.g.out_planes && store_mode() && (src.g.out_nb32 & 1) == 0 &&
-            ((reinterpret_cast<uintptr_t>(src.g.out) | reinterpret_cast<uintptr_t>(src.g.out_lo)) & 127) == 0) {
-          if ((rc = make_store_map(&pr.o_hi, src.g.out, src.g.M, src.g.out_nb32 / 2))) return rc;
-          if ((rc = make_store_map(&pr.o_lo, src.g.out_lo, src.g.M, src.g.out_nb32 / 2))) return rc;
-          pr.g.out_tma = 1;
-        }
-        pr.g.a_mn = src.a.mn_major;
-        pr.g.b_mn = src.b.mn_major;
-        pr.g.tiles_m = (int)ceil_div(pr.g.M, tm);
-        pr.g.tiles_n = (int)ceil_div(pr.g.N, tn);
-        pr.g.tiles = pr.g.tiles_m * pr.g.tiles_n;
-        if ((int64_t)pr.g.tiles * pr.g.splits >= (1 << 21))
-          return fail(ADN_ERR_UNSUPPORTED, "%s: %d work items exceed the decode range", what, pr.g.tiles * pr.g.splits);
-        pr.g.inv_tiles = 1.0f / (float)pr.g.tiles;
-        pr.g.inv_tiles_n = 1.0f / (float)pr.g.tiles_n;
-        pr.g.inv_tiles_m = 1.0f / (float)pr.g.tiles_m;
-        pr.g.m_fastest = item_order_m_fastest(pr.g);
-        pr.g.ovf = g_ovf_addr;
-        pr.item0 = items;
-        items += pr.g.tiles_m * pr.g.tiles_n * pr.g.splits;
+  for (int i0 = 0; i0 < n; i0 += MAX_GROUP) {
+    const int m = std::min(MAX_GROUP, n - i0);
+    Group grp;
+    memset(&grp, 0, sizeof(grp));
+    int items = 0;
+    for (int i = 0; i < m; ++i) {
+      const GemmDesc& src = d[i0 + i];
+      Problem& pr = grp.p[i];
+      int rc = encode_maps(fmt, src, &pr.a_hi, &pr.a_lo, &pr.b_hi, &pr.b_lo, what);
+      if (rc) return rc;
+      pr.g = src.g;
+      pr.g.out_tma = 0;
+      if (fmt == FMT_F16 && EPI != EPI_PARTIAL && src.g.out_planes && (src.g.out_nb32 & 1) == 0 &&
+          ((reinterpret_cast<uintptr_t>(src.g.out) | reinterpret_cast<uintptr_t>(src.g.out_lo)) & 127) == 0) {
+        if ((rc = make_store_map(&pr.o_hi, src.g.out, src.g.M, src.g.out_nb32 / 2))) return rc;
+        if ((rc = make_store_map(&pr.o_lo, src.g.out_lo, src.g.M, src.g.out_nb32 / 2))) return rc;
+        pr.g.out_tma = 1;
       }
-      grp.n = m;
-      grp.total_items = items;
-      if (pair) {
-        const int grid = 2 * std::min(items, sm_count() / 2);
-        if (fmt == FMT_F16) launch_kernel2<FMT_F16, EPI>(grp, grid, st);
-        else launch_kernel2<FMT_TF32, EPI>(grp, grid, st);
-      } else {
-        const int grid = std::min(items, sm_count());
-        if (fmt == FMT_F16) launch_kernel<FMT_F16, EPI>(grp, grid, st);
-        else launch_kernel<FMT_TF32, EPI>(grp, grid, st);
-      }
-      ADN_CHECK_LAUNCH(what);
+      pr.g.a_mn = src.a.mn_major;
+      pr.g.b_mn = src.b.mn_major;
+      pr.g.tiles_m = (int)ceil_div(pr.g.M, BM);
+      pr.g.tiles_n = (int)ceil_div(pr.g.N, BN);
+      pr.g.tiles = pr.g.tiles_m * pr.g.tiles_n;
+      if ((int64_t)pr.g.tiles * pr.g.splits >= (1 << 21))
+        return fail(ADN_ERR_UNSUPPORTED, "%s: %d work items exceed the decode range", what, pr.g.tiles * pr.g.splits);
+      pr.g.inv_tiles = 1.0f / (float)pr.g.tiles;
+      pr.g.inv_tiles_n = 1.0f / (float)pr.g.tiles_n;
+      pr.g.ovf = g_ovf_addr;
+      pr.item0 = items;
+      items += pr.g.tiles_m * pr.g.tiles_n * pr.g.splits;
     }
+    grp.n = m;
+    grp.total_items = items;
+    const int grid = std::min(items, sm_count());
+    if (fmt == FMT_F16) launch_kernel<FMT_F16, EPI>(grp, grid, st);
+    else launch_kernel<FMT_TF32, EPI>(grp, grid, st);
+    ADN_CHECK_LAUNCH(what);
   }
   return ADN_OK;
 }
@@ -1715,15 +1290,14 @@ int dense_bwd_group(int fmt, const BwdOp* ops, int n, int64_t batch, cudaStream_
       const double kItemOverhead = 6.0;          // k-block equivalents per work item
       const double kReduceKbPerByte = 1.0 / (2.5e6 * 0.4);     // k-block equivalents per byte of partials read
       double best_t = 1e30;
-      std::vector<double> load((size_t)workers), load2((size_t)std::max(1, workers / 2));
+      std::vector<double> load((size_t)workers);
       int64_t last_kps = -1;
       for (int s0 = 1; s0 <= MAX_SPLITS && s0 <= kb_b; ++s0) {
         const int64_t kps = ceil_div(kb_b, s0);
         if (kps == last_kps) continue;
         last_kps = kps;
         std::fill(load.begin(), load.end(), 0.0);
-        std::fill(load2.begin(), load2.end(), 0.0);
-        int64_t item = 0, item2 = 0;
+        int64_t item = 0;
         double reduce_bytes = 0.0;
         bool any = false;
         for (int i = 0; i < n; ++i) {
@@ -1731,24 +1305,16 @@ int dense_bwd_group(int fmt, const BwdOp* ops, int n, int64_t batch, cudaStream_
           any = true;
           const int64_t k_i = std::max<int64_t>(kps, ceil_div(kb_b, max_dw_splits(ops[i].in, ops[i].out)));
           const int64_t s_i = ceil_div(kb_b, k_i);
-          // problems on the CTA-pair kernel run as their own launch: 256x256 tiles on SM pairs, twice the tensor
-          // work per k-block and tile
-          const bool pair = use_pair_shape(fmt, ops[i].in, ops[i].out, kb_b);
-          const int64_t tiles = pair ? ceil_div(ops[i].in, BM2) * ceil_div(ops[i].out, BN2)
-                                     : ceil_div(ops[i].in, BM) * ceil_div(ops[i].out, BN);
+          const int64_t tiles = ceil_div(ops[i].in, BM) * ceil_div(ops[i].out, BN);
           for (int64_t sp = 0; sp < s_i; ++sp) {
             const double kb_item = (double)(std::min(kb_b, (sp + 1) * k_i) - sp * k_i);
-            if (pair) {
-              for (int64_t t = 0; t < tiles; ++t, ++item2) load2[(size_t)(item2 % (int64_t)load2.size())] += 2.0 * (kb_item + kItemOverhead);
-            } else {
-              for (int64_t t = 0; t < tiles; ++t, ++item) load[(size_t)(item % workers)] += kb_item + kItemOverhead;
-            }
+            for (int64_t t = 0; t < tiles; ++t, ++item) load[(size_t)(item % workers)] += kb_item + kItemOverhead;
           }
           if (s_i > 1) reduce_bytes += (double)(s_i + 1) * (double)ops[i].in * (double)ops[i].out * 4.0;
         }
         if (!any) break;
-        const double t = *std::max_element(load.begin(), load.end()) + *std::max_element(load2.begin(), load2.end()) +
-                         reduce_bytes * kReduceKbPerByte + (reduce_bytes > 0 ? 10.0 : 0.0);
+        const double t = *std::max_element(load.begin(), load.end()) + reduce_bytes * kReduceKbPerByte +
+                         (reduce_bytes > 0 ? 10.0 : 0.0);
         if (t < best_t) { best_t = t; best_kps = kps; }
       }
       std::lock_guard<std::mutex> lk(mu);

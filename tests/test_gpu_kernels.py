@@ -263,7 +263,6 @@ def test_conv_stem_fwd_bwd(gpu, monkeypatch, conv_path, B, H, W, CIN, F):
   import torch
   from adanet_b200 import _lib
   monkeypatch.setenv("ADN_CONV_PATH", conv_path)
-  monkeypatch.setenv("ADN_CONV_BWD_PATH", conv_path)      # the backward's tcgen05 variant is opt-in
   rng = np.random.default_rng(B * 7 + H + F)
   x = rng.uniform(0, 1, (B, H, W, CIN)).astype(np.float32)
   k = (rng.standard_normal((3, 3, CIN, F)) * np.sqrt(2.0 / (9 * CIN))).astype(np.float32)   # he_normal scale
